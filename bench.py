@@ -2,6 +2,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one rank per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W    # the CPU restatement of the reference path, host cores
+    python bench.py --steps K --dump-outputs DIR             # + the last timed step's TimeStep as DIR/<name>.npy
 
 One "step" = one `Environment.step` for the whole batch = n_sub_steps(5) physics steps + reward + observation
 (reference: rl/control.py:99-127, suite/humanoid.py:30). Prints ONE JSON line on rank 0. See DESIGN.md §Measurement.
@@ -19,6 +20,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: the benchmark leaves it as it found it
 
 METRIC = 'env-steps/sec suite.humanoid:run batch 8192 (per GPU) random-action rollout'
 UNIT = 'env-steps/s'
@@ -166,7 +168,8 @@ def time_cpu(total_envs=BATCH, warmup_steps=21, reps=3, target_s=3.0):
   2. one pinned process per physical core, the BATCH environments split evenly (capped so that a window stays near
      `target_s` seconds of work per process), `reps` timed windows, each started at a barrier; a window's time is the
      span from the first start to the last finish; the best window is reported.
-  Returns a dict (value = env-steps/s of the best window)."""
+  The window is sized here, not by --steps: the scalar host path would need minutes for --steps x 8192 environments.
+  Returns a dict (value = env-steps/s of the best window, steps = env-steps each timed window ran)."""
   from oracle import oracle as om
   om.build()
   cores = physical_cores()
@@ -185,7 +188,7 @@ def time_cpu(total_envs=BATCH, warmup_steps=21, reps=3, target_s=3.0):
     rates.append(nenv * len(cores) * timed / dt)
   best = max(rates)
   single = 1e6 / (us_per_phys * NSUB)                          # env-steps/s of one core alone
-  return dict(value=best, unit=UNIT, cores=len(cores), kind='port',
+  return dict(value=best, unit=UNIT, cores=len(cores), kind='port', steps=timed,
               sample=(f'{nenv * len(cores)} envs ({nenv}/process x {len(cores)} processes, one pinned per physical core) x {timed} '
                       f'env-steps x {reps} windows (best) after {warmup_steps} settle steps, seeded humanoid:run states, uniform(-1,1) actions'),
               per_core_us_per_physics_step=us_per_phys, parallel_efficiency=best / (single * len(cores)),
@@ -203,8 +206,9 @@ def run_reference(args):
     sys.path.insert(0, os.path.join(ROOT, 'tools'))
     import time_mujoco_cpu
     if time_mujoco_cpu.available():      # a machine that has the real reference: time that instead
-      value, cores, sample, ms = time_mujoco_cpu.time_reference(21, max(20, min(args.steps, 300)), 8)
-      cpu = dict(value=value, unit=UNIT, cores=cores, kind='reference', sample=sample, ms_per_env_step_batch=ms)
+      ref_steps = max(20, min(args.steps, 300))
+      value, cores, sample, ms = time_mujoco_cpu.time_reference(21, ref_steps, 8)
+      cpu = dict(value=value, unit=UNIT, cores=cores, kind='reference', steps=ref_steps, sample=sample, ms_per_env_step_batch=ms)
       kind, note = 'reference', 'unmodified dm_control suite.load(humanoid, run) on mujoco, Environment.step'
   except Exception as ex:
     sys.stderr.write(f'real-reference arm failed ({ex!r}); timing the oracle port\n')
@@ -212,7 +216,7 @@ def run_reference(args):
   if cpu is None:
     cpu = time_cpu()
   value = cpu['value']
-  line = dict(impl='reference', metric=METRIC, value=value, unit=UNIT, n_gpus=args.gpus, steps=args.steps, warmup=args.warmup,
+  line = dict(impl='reference', metric=METRIC, value=value, unit=UNIT, n_gpus=args.gpus, steps=cpu['steps'], warmup=args.warmup,
               ms_per_step=cpu.pop('ms_per_env_step_batch'), higher_is_better=True, scaling='weak', vs_baseline=None, dtype='f64',
               data='synthetic',
               config=dict(workload='suite.humanoid:run', batch_per_gpu=BATCH, n_sub_steps=NSUB, note=note),
@@ -248,7 +252,7 @@ def _time_env(env, steps, warmup, gen_seed, nu, dev):
   e1.record(); torch.cuda.synchronize(dev)
   ms = e0.elapsed_time(e1) / steps
   d = env.physics.data
-  return dict(batch=B, n_sub_steps=env.n_sub_steps, ms_per_step=ms, env_steps_per_s=B / ms * 1e3,
+  return dict(batch=B, n_sub_steps=env.n_sub_steps, steps=steps, ms_per_step=ms, env_steps_per_s=B / ms * 1e3,
               physics_steps_per_s=B * env.n_sub_steps / ms * 1e3, mean_ncon=_mean_ncon(d),
               warnings=[int(x) for x in d.warning.sum(0).tolist()])
 
@@ -263,6 +267,18 @@ def _contact_load(snaps, caps):
   return dict(mean_ncon=float(ncon.mean()), mean_nefc=float(nefc.mean()), p99_nefc=float(torch.quantile(nefc, 0.99)),
               max_nefc=float(nefc.max()), mean_niter=float(niter.mean()), bucket_caps=list(caps), bucket_populations=pops,
               note='state after each sampled env-step: ncon / nefc of the trailing mj_step1, solver iterations of its last physics step')
+
+
+def dump_outputs(out_dir, ts):
+  """The TimeStep of the last timed env.step as DIR/<name>.npy (float64): step_type, reward, discount and one file per
+  observation (observation.<key>). For batch 8192 that is ~4.6 MB, so nothing is sampled."""
+  import numpy as np
+  import torch
+  os.makedirs(out_dir, exist_ok=True)
+  arrays = dict(step_type=ts.step_type, reward=ts.reward, discount=ts.discount)
+  arrays.update({f'observation.{k}': v for k, v in ts.observation.items()})
+  for name, t in arrays.items():
+    np.save(os.path.join(out_dir, name + '.npy'), t.detach().to('cpu', dtype=torch.float64).numpy())
 
 
 def run_gpu(args):
@@ -399,10 +415,12 @@ def run_gpu(args):
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
+    ts = None
     for i in range(steps):
       flush.fill_(0.0)
       actions.copy_(act_tape[i % len(act_tape)], non_blocking=True)     # H2D from pinned host memory
-      pack(env.step(actions))
+      ts = env.step(actions)
+      pack(ts)
       out_host.copy_(packed, non_blocking=True)                         # D2H of this rank's rows
       torch.cuda.current_stream().synchronize()                         # the user reads obs before the next action
     e1.record()
@@ -410,9 +428,11 @@ def run_gpu(args):
     tt = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
     if world > 1:
       dist.all_reduce(tt, op=dist.ReduceOp.MAX)
-    return batch * world * steps / (float(tt[0]) * 1e-3)
+    return batch * world * steps / (float(tt[0]) * 1e-3), ts
 
-  e2e_value = e2e(env, BATCH, actions, packed, gathered, pack, world, args.steps)
+  e2e_value, last_ts = e2e(env, BATCH, actions, packed, gathered, pack, world, args.steps)
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, last_ts)
   warn = phys.data.warning.sum(0)
   if world > 1:
     dist.all_reduce(warn)
@@ -435,7 +455,7 @@ def run_gpu(args):
     dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     strong = dict(global_batch=BATCH, batch_per_gpu=sb, value=BATCH * args.steps / (float(tt[0]) * 1e-3), unit=UNIT,
                   ms_per_step=float(tt[0]) / args.steps,
-                  e2e=e2e(env_s, sb, actions_s, packed_s, gathered_s, pack_s, world, args.steps))
+                  e2e=e2e(env_s, sb, actions_s, packed_s, gathered_s, pack_s, world, args.steps)[0])
 
   # ---- the other BASELINE.json configs on one GPU, same run (device-resident, through env.step) ---------------
   configs = None
@@ -444,18 +464,18 @@ def run_gpu(args):
     for dom, task, B in (('cheetah', 'run', 4096), ('quadruped', 'walk', 4096), ('cartpole', 'swingup', 4096)):
       try:
         e = suite.load(dom, task, batch=B, seed=3, device=dev)
-        configs[f'suite.{dom}:{task}'] = _time_env(e, 20, 10, 5, e.physics.model.nu, dev)
+        configs[f'suite.{dom}:{task}'] = _time_env(e, args.steps, 10, 5, e.physics.model.nu, dev)
         e.physics.free()
       except Exception as ex:
         configs[f'suite.{dom}:{task}'] = dict(error=repr(ex))
     try:
       from dm_control_b200 import locomotion
       e = locomotion.load('cmu_humanoid_run_walls', batch=2048, seed=3, device=dev)
-      configs['locomotion.cmu_humanoid run-through-corridor (walls)'] = _time_env(e, 10, 10, 5, e.physics.model.nu, dev)
+      configs['locomotion.cmu_humanoid run-through-corridor (walls)'] = _time_env(e, args.steps, 10, 5, e.physics.model.nu, dev)
       e.physics.free()
       # the same with the walker's 64 x 64 egocentric camera observable, ray-cast on the device every control step (b200mj_render)
       e = locomotion.load('cmu_humanoid_run_walls', batch=2048, seed=3, device=dev, egocentric_camera=True)
-      r = _time_env(e, 10, 10, 5, e.physics.model.nu, dev)
+      r = _time_env(e, args.steps, 10, 5, e.physics.model.nu, dev)
       r['observation'] = 'walker/egocentric_camera [2048, 64, 64, 3] uint8 per step (ray-cast hand-off, not MuJoCo GL pixels)'
       configs['locomotion.cmu_humanoid run-through-corridor (walls) + egocentric camera'] = r
       e.physics.free()
@@ -516,7 +536,10 @@ def main():
   ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
   ap.add_argument('--no-cpu', action='store_true', help='skip the cpu_baseline leg')
   ap.add_argument('--no-configs', action='store_true', help='skip the other BASELINE.json configs (N=1 only)')
+  ap.add_argument('--dump-outputs', metavar='DIR', help='write the TimeStep of the last timed step (rank 0) as DIR/<name>.npy')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
   if args.impl == 'reference':
     run_reference(args)
   else:

@@ -1,13 +1,14 @@
 """north_star: "suite tasks run unchanged". The UNMODIFIED reference sources — dm_control/rl/control.py (Environment),
 dm_control/suite/{humanoid,cartpole,cheetah,quadruped}.py (tasks + Physics subclasses, incl. the model editing cartpole.py
 and quadruped.py do with lxml), suite/base.py, suite/common, suite/utils/randomizers.py, utils/rewards.py,
-utils/containers.py, utils/xml_tools.py — are imported from /root/reference (tests/refshim wires the few absent
-third-party modules) and drive a B = 1 view of the batched CUDA engine (dm_control_b200/refview.py): humanoid:run for 100
-control steps, the other BASELINE suite configs and eight further domains for 20 (tools/probe_reference_suite.py sweeps all 47
-tasks of the reference suite: 30 run, 17 are refused for a named unsupported feature). The trajectory is checked against the CPU oracle stepped from the
-same post-reset state with the same actions.
+utils/containers.py, utils/xml_tools.py — drove a B = 1 view of the batched CUDA engine (dm_control_b200/refview.py,
+tests/refshim wires the few absent third-party modules): humanoid:run for 100 control steps, the other BASELINE suite
+configs and eight further domains for 20 (tools/probe_reference_suite.py sweeps all 47 tasks of the reference suite: 30
+run, 17 are refused for a named unsupported feature). tools/make_reference_goldens.py stored, per task, the model the
+task file built, the state its `reset` left, and what the run saw step by step, in tests/golden/reference_tasks.npz.
 
-/root/reference exists in the build container only: the tests skip where it is absent (GPU box).
+Here the engine is stepped from that state on that model with the same seeded actions, and checked against the CPU
+oracle stepped alongside and against the stored contact counts:
   * `-m gpu` twin: runs on the device (or under B200MJ_EMULATE_GPU=1);
   * CPU-collectable test: runs the same body in a child process against the CPU emulation build of the kernels."""
 import os
@@ -18,84 +19,88 @@ import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, 'tests'))
-import refshim   # noqa: E402
+GOLD = os.path.join(ROOT, 'tests', 'golden', 'reference_tasks.npz')
 
-needs_reference = pytest.mark.skipif(not refshim.available(), reason='/root/reference is not on this machine')
+
+def _replay(domain, task):
+  """-> (B = 1 view, oracle, stored run, actions) of `domain:task`: view and oracle both start from the state the
+  reference's `reset` left; the actions are the run's seeded uniform draws within the action spec."""
+  import io
+  from dm_control_b200 import refview
+  from dm_control_b200.model import Model
+  from oracle import oracle as om
+  name = f'{domain}_{task}'
+  with np.load(GOLD) as z:
+    run = {k[len(name) + 1:]: z[k] for k in z.files if k.startswith(name + '/')}
+    model = Model.load(io.BytesIO(z['model/' + str(run['model'])].tobytes()))
+  phys = refview.SingleEnvPhysics(model)
+  start = {k[len('start_'):]: v for k, v in run.items() if k.startswith('start_')}     # absent: zero, as the view starts
+  for k, v in start.items():
+    np.copyto(phys.data._arrays[k], v)
+  o = om.OraclePhysics(model)
+  o.qpos[:] = start.get('qpos', 0.0); o.qvel[:] = start.get('qvel', 0.0)
+  if model.na:
+    o.act[:] = start.get('act', 0.0)
+  o.forward()
+  (action_seed, nsteps), = [(a, n) for d, t, _, a, n in RUNS if (d, t) == (domain, task)]
+  rs = np.random.RandomState(action_seed)
+  actions = [rs.uniform(run['action_minimum'], run['action_maximum']) for _ in range(nsteps)]
+  return phys, o, run, actions
 
 
 def run_unmodified_humanoid(nsteps=100):
-  refshim.install()
-  import dm_control.suite.humanoid as ref_humanoid            # the reference file itself
-  assert os.path.realpath(ref_humanoid.__file__).startswith(os.path.realpath(refshim.REFERENCE))
-  from oracle import oracle as om
-  env = ref_humanoid.run(random=7)                            # control.Environment(Physics, Humanoid, ...), unmodified
-  spec = env.action_spec()
-  assert spec.shape == (21,) and spec.minimum.min() == -1 and spec.maximum.max() == 1
-  ts = env.reset()
-  assert ts.first() and ts.reward is None
-  assert env.physics.data.ncon == 0                           # humanoid.py:160-166: re-drawn until contact-free
-  assert set(ts.observation) == {'joint_angles', 'head_height', 'extremities', 'torso_vertical', 'com_velocity', 'velocity'}
-  phys = env.physics
-  o = om.OraclePhysics(phys.model)
-  o.qpos[:] = phys.data.qpos; o.qvel[:] = phys.data.qvel; o.forward()
-  rs = np.random.RandomState(3)
+  phys, o, run, actions = _replay('humanoid', 'run')
+  assert o.ncon == 0                                          # humanoid.py:160-166: re-drawn until contact-free
+  assert _batched_observation_keys('humanoid', 'run') == [str(k) for k in run['observation_keys']] == sorted(
+      ['joint_angles', 'head_height', 'extremities', 'torso_vertical', 'com_velocity', 'velocity'])
+  nsub = int(run['n_sub_steps'])
   worst = 0.0
-  for t in range(nsteps):
-    a = rs.uniform(-1, 1, 21)
-    ts = env.step(a)
-    o.ctrl[:] = a; o.control_step(5)                          # control_timestep .025 / timestep .005
-    assert not ts.last() and ts.discount == 1.0
-    assert 0.0 <= ts.reward <= 1.0
+  for t, a in enumerate(actions):
+    phys.set_control(a); phys.step(nsub)                      # what control.Environment.step does to the physics
+    o.ctrl[:] = a; o.control_step(nsub)
     worst = max(worst, float(np.abs(phys.data.qpos - o.qpos).max()), float(np.abs(phys.data.qvel - o.qvel).max()) * 0.1)
-    assert phys.data.ncon == o.ncon
+    assert phys.data.ncon == o.ncon == run['ncon'][t]
     assert [(c.geom1, c.geom2) for c in phys.data.contact] == [(c.geom1, c.geom2) for c in o.contact]
     # the reference task's own observation code, on the oracle's numbers
-    np.testing.assert_allclose(ts.observation['joint_angles'], o.qpos[7:], atol=1e-6)
-    np.testing.assert_allclose(ts.observation['head_height'], np.asarray(o.xpos).reshape(-1, 3)[phys.model.name2id('head', 'body'), 2], atol=1e-6)
-  assert abs(env.physics.time() - nsteps * 0.025) < 1e-9
+    np.testing.assert_allclose(run['joint_angles'][t], o.qpos[7:], atol=1e-6)
+    np.testing.assert_allclose(run['head_height'][t], np.asarray(o.xpos).reshape(-1, 3)[phys.model.name2id('head', 'body'), 2], atol=1e-6)
+  assert abs(phys.time() - nsteps * 0.025) < 1e-9
   assert worst < 1e-6, worst
   return worst
 
 
-def run_unmodified(domain, task, nsteps=20, seed=5):
-  """Any of the BASELINE suite configs through the reference's own task file: build (the file's own model editing where it
-  has any: cartpole.py:104-127, quadruped.py:55-93), reset (its own randomisation), step with random actions; the
-  trajectory against the oracle stepped from the same post-reset state. Convex (MPR) contacts end the comparison of an
-  episode (DESIGN.md 3: discontinuous in the pose)."""
-  import importlib
-  refshim.install()
-  mod = importlib.import_module('dm_control.suite.' + domain)
-  assert os.path.realpath(mod.__file__).startswith(os.path.realpath(refshim.REFERENCE))
-  from oracle import oracle as om
-  env = getattr(mod, task)(random=seed)
-  spec = env.action_spec()
-  ts = env.reset()
-  assert ts.first() and ts.reward is None
-  phys = env.physics
-  nsub = int(round(env.control_timestep() / phys.timestep()))
-  o = om.OraclePhysics(phys.model)
-  o.qpos[:] = phys.data.qpos; o.qvel[:] = phys.data.qvel
-  if phys.model.na:
-    o.act[:] = phys.data.act
-  o.forward()
+def _batched_observation_keys(domain, task):
+  """Observation keys of this repo's batched twin of the task."""
+  from dm_control_b200 import suite as bsuite
+  return sorted(bsuite.load(domain, task, batch=1, seed=0).reset().observation)
+
+
+def run_unmodified(domain, task, batched=False):
+  """Any of the BASELINE suite configs as the reference's own task file ran it: built (the file's own model editing where
+  it has any: cartpole.py:104-127, quadruped.py:55-93), reset (its own randomisation), stepped with random actions;
+  the engine against the oracle stepped from the same post-reset state. Convex (MPR) contacts end the comparison of an
+  episode (DESIGN.md 3: discontinuous in the pose). `batched`: the task has a batched twin here, whose observation
+  keys must be the reference task's."""
+  phys, o, run, actions = _replay(domain, task)
+  nsub = int(run['n_sub_steps'])
   gtype = np.asarray(phys.model.geom_type)
-  rs = np.random.RandomState(11)
   worst, compared = 0.0, 0
-  for t in range(nsteps):
-    a = rs.uniform(spec.minimum, spec.maximum)
-    ts = env.step(a)
+  for t, a in enumerate(actions):
+    phys.set_control(a); phys.step(nsub)
     o.ctrl[:] = a; o.control_step(nsub)
-    assert ts.reward is not None and 0.0 <= ts.reward <= 1.0 + 1e-12
     if any(gtype[c.geom1] != 0 and (gtype[c.geom1] > 3 or gtype[c.geom2] > 3) for c in o.contact):
       break
     worst = max(worst, float(np.abs(phys.data.qpos - o.qpos).max()), float(np.abs(phys.data.qvel - o.qvel).max()) * 0.1)
-    assert phys.data.ncon == o.ncon
+    assert phys.data.ncon == o.ncon == run['ncon'][t]
     assert [(c.geom1, c.geom2) for c in phys.data.contact] == [(c.geom1, c.geom2) for c in o.contact]
     compared += 1
-  assert abs(env.physics.time() - (t + 1) * env.control_timestep()) < 1e-9
-  assert compared >= min(10, nsteps) and worst < 1e-6, (compared, worst)
-  return dict(worst=worst, compared=compared, nsub=nsub, obs=sorted(ts.observation))
+  assert abs(phys.time() - (t + 1) * nsub * phys.timestep()) < 1e-9
+  assert compared >= min(10, len(actions)) and worst < 1e-6, (compared, worst)
+  out = dict(worst=worst, compared=compared, nsub=nsub)
+  if batched:
+    out['obs'] = _batched_observation_keys(domain, task)
+    assert out['obs'] == [str(k) for k in run['observation_keys']], (out['obs'], run['observation_keys'])
+  return out
 
 
 _SUITE_CASES = [
@@ -110,19 +115,21 @@ _SUITE_CASES = [
     ('point_mass', 'hard', None),         # writes physics.model.wrap_prm in place (point_mass.py:101-112)
     ('reacher', 'hard', None), ('walker', 'run', None), ('cartpole', 'three_poles', None),
 ]
+# the stored runs: (domain, task, the task's random seed, the seed of the uniform actions, control steps)
+RUNS = [('humanoid', 'run', 7, 3, 100)] + [(d, t, 5, 11, 20) for d, t, _ in _SUITE_CASES]
 
 
 @pytest.fixture(scope='module')
 def emulated_suite_results():
   """ONE child process (CPU emulation build of the kernels) runs every case; the parametrized tests read their entry."""
   import json
-  cases = [(d, t) for d, t, _ in _SUITE_CASES]
+  cases = [(d, t, keys is not None) for d, t, keys in _SUITE_CASES]
   code = ("import os, sys, json, traceback; sys.path.insert(0, %r); sys.path.insert(0, %r); sys.path.insert(0, %r);"
           "import gpu_shim; gpu_shim.install();"
           "import test_reference_tasks as t\n"
           "out = {}\n"
-          "for d, k in %r:\n"
-          "  try: out[d + ':' + k] = t.run_unmodified(d, k)\n"
+          "for d, k, b in %r:\n"
+          "  try: out[d + ':' + k] = t.run_unmodified(d, k, b)\n"
           "  except BaseException as ex: out[d + ':' + k] = dict(error=traceback.format_exc()[-1500:])\n"
           "print('RESULT', json.dumps(out))") % (ROOT, os.path.join(ROOT, 'tests'), os.path.join(ROOT, 'tests', 'emu'), cases)
   env = dict(os.environ, B200MJ_EMULATE_GPU='1')
@@ -131,10 +138,9 @@ def emulated_suite_results():
   return json.loads(r.stdout.split('RESULT', 1)[1])
 
 
-@needs_reference
 @pytest.mark.parametrize('domain,task,keys', _SUITE_CASES)
 def test_unmodified_reference_suite_tasks_under_emulation(domain, task, keys, emulated_suite_results):
-  """The reference's own suite/<domain>.py drives the engine (CPU emulation build of the kernels, child process)."""
+  """The engine on what the reference's own suite/<domain>.py built and drove (CPU emulation build of the kernels, child process)."""
   out = emulated_suite_results[f'{domain}:{task}']
   assert 'error' not in out, out.get('error')
   assert out['compared'] >= 10 and out['worst'] < 1e-6, out
@@ -142,13 +148,11 @@ def test_unmodified_reference_suite_tasks_under_emulation(domain, task, keys, em
     assert out['obs'] == sorted(keys), out
 
 
-@needs_reference
 @pytest.mark.gpu
 def test_unmodified_reference_humanoid_task_on_the_engine():
   run_unmodified_humanoid(100)
 
 
-@needs_reference
 def test_unmodified_reference_humanoid_task_under_emulation():
   """CPU-collectable twin: the same body in a child process, kernels from the CPU emulation build (tests/emu)."""
   code = ("import os, sys; sys.path.insert(0, %r); sys.path.insert(0, %r); sys.path.insert(0, %r);"
